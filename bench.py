@@ -6,7 +6,7 @@ reference's own `model(x)` protocol), roofline entries for every kernel kind >= 
 check of the timed batch against the fp32 oracle, the other BASELINE configs, and the reference's CPU path
 timed beside it.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One JSON line on stdout (rank 0).  "step" = one forward of `batch` images per GPU (weak scaling:
@@ -58,7 +58,36 @@ def parse_args():
     ap.add_argument("--no-configs", action="store_true", help="skip the other BASELINE configs (C1, C4, C5)")
     ap.add_argument("--no-parity", action="store_true")
     ap.add_argument("--no-two-in-flight", action="store_true", help="skip the two-handles / two-threads end-to-end extra")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned (rank 0: logits, ids, steps) to DIR/<name>.npy as float32")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the engine's outputs: it needs --impl ours")
+    return args
+
+
+DUMP_MAX_BYTES = 64_000_000
+
+
+def dump_outputs(out_dir, logits, ids, steps):
+    """The arrays the caller of the timed path receives, as float32 .npy files (ids <= 96 and the step count are exact).
+    When the batch is too large for DUMP_MAX_BYTES, a fixed seeded sample of rows is written with its row indices."""
+    import numpy as np
+    import torch
+    B = logits.shape[0]
+    row_bytes = (logits[0].numel() + ids[0].numel()) * 4
+    arrays = {"logits": logits, "ids": ids}
+    if B * row_bytes > DUMP_MAX_BYTES:
+        n = (DUMP_MAX_BYTES - 4096) // (row_bytes + 4)          # + its row index; 4 KB for the .npy headers
+        rows = torch.randperm(B, generator=torch.Generator().manual_seed(0))[:n].sort().values
+        arrays = {k: v.cpu()[rows] for k, v in arrays.items()}
+        arrays["rows"] = rows
+    arrays["steps"] = steps
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().cpu().to(torch.float32).numpy())
 
 
 def load_peaks():
@@ -460,6 +489,8 @@ def main():
     ms = e0.elapsed_time(e1)
     launches = eng.launches - l0
     last_batch = (args.steps - 1) % NROT
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, logits, ids, steps_t)
     if distributed:
         t = torch.tensor([ms], device=dev)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)

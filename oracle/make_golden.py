@@ -2,7 +2,7 @@
 (/root/reference/strhub/models/parseq/model.py under oracle/timm_shim.py) on seeded synthetic
 weights and crops.  Run in the build container (the GPU box has no /root/reference):
 
-    python -m oracle.make_golden
+    python -m oracle.make_golden [vitstr | sharp | reference | filtered ...]
 
 TEST INFRASTRUCTURE ONLY.  Weights are not stored: they are regenerated from (experiment, seed) by
 parseq_b200.weights.init_state_dict and verified through `sd_digest`.
@@ -184,9 +184,50 @@ def make_vitstr():
         print(f"{name:18s} logits {tuple(logits.shape)} |ref-fp64 oracle|={err:.2e}")
 
 
+def make_reference_surface():
+    """tests/golden/reference/: what the CPU tests compare against that is not a forward case of CASES — the reference
+    PARSeq-Ti on one (weights, crops) pair under three decode schedules, the reference state_dict layout, and the
+    reference Tokenizer on fixed inputs."""
+    from parseq_b200.config import CHARSET_94
+    out = os.path.join(OUT, "reference")
+    os.makedirs(out, exist_ok=True)
+    cfg, sd = make_sd("parseq-tiny", 11, 0.0)
+    ref, tok = RL.build_reference_model(cfg, sd)
+    x = synth_images(cfg, 2, 12)
+    runs = []
+    for ar, ri, ml in [(True, 1, None), (False, 0, None), (True, 2, 4)]:
+        ref.decode_ar, ref.refine_iters = ar, ri
+        with torch.inference_mode():
+            runs.append(dict(decode_ar=ar, refine_iters=ri, max_length=ml, logits=ref(tok, x, ml).clone()))
+    torch.save(dict(experiment="parseq-tiny", weight_seed=11, batch=2, image_seed=12, sd_digest=state_dict_digest(sd), runs=runs,
+                    source="reference strhub.models.parseq.model.PARSeq (timm shim), torch %s CPU fp32" % torch.__version__),
+               os.path.join(out, "tiny_w11_x12.pt"))
+
+    cfg, sd = make_sd("parseq", 0, 0.0)
+    ref, _ = RL.build_reference_model(cfg, sd)          # strict load
+    shapes = {k: tuple(v.shape) for k, v in ref.state_dict().items()}
+    _, RefTok = RL.load_reference_classes()
+    rt = RefTok(CHARSET_94)
+    # probabilities with a clear argmax per position: ids 11 12 | EOS 13 14 and 37 1 2 3 4 (no EOS)
+    probs = torch.zeros(2, 5, 95)
+    for b, seq in enumerate([[11, 12, 0, 13, 14], [36 + 1, 1, 2, 3, 4]]):
+        for i, t in enumerate(seq):
+            probs[b, i, t] = 0.9
+    labels, ps = rt.decode(probs)
+    texts = ["ab", "hello!"]
+    torch.save(dict(state_dict_shapes=shapes, charset=CHARSET_94, decode_probs=probs, decode_labels=labels,
+                    decode_token_probs=[p.clone() for p in ps], encode_texts=texts, encode_ids=rt.encode(texts),
+                    source="reference strhub.models.parseq.model.PARSeq / strhub.data.utils.Tokenizer, torch %s"
+                           % torch.__version__),
+               os.path.join(out, "surface.pt"))
+    print("reference surface:", len(shapes), "state_dict entries,", len(runs), "PARSeq-Ti runs")
+
+
 if __name__ == "__main__":
     if len(sys.argv) > 1 and sys.argv[1] == "vitstr":
         make_vitstr()
+    elif len(sys.argv) > 1 and sys.argv[1] == "reference":
+        make_reference_surface()
     elif len(sys.argv) > 1 and sys.argv[1] == "sharp":
         main(SHARP_CASES)
     elif len(sys.argv) > 1 and sys.argv[1] == "filtered_ti":

@@ -1,9 +1,9 @@
-"""Imports the reference's own `strhub.models.parseq.model.PARSeq` from /root/reference (read-only,
-present in the build container only) under the timm shim.  TEST INFRASTRUCTURE ONLY: used by
-oracle/make_golden.py and by CPU tests that are skipped when /root/reference is absent.
+"""Imports the reference's own `strhub.models.parseq.model.PARSeq` from the reference tree (REF_ROOT, read-only)
+under the timm shim.  TEST INFRASTRUCTURE ONLY: used by oracle/make_golden.py, which stores the reference's outputs
+under tests/golden; the tests compare against those and never import the reference.
 
-On the GPU box /root/reference does not exist: there the byte-compiled copy `oracle/_ref/` (oracle/build_ref.py) is
-imported instead, and only by bench.py's CPU legs (`--impl reference`, `cpu_baseline`).
+Where the reference tree is absent, the byte-compiled copy `oracle/_ref/` (oracle/build_ref.py) is imported instead,
+and only by bench.py's CPU legs (`--impl reference`, `cpu_baseline`).
 """
 from __future__ import annotations
 
