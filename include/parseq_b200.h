@@ -103,11 +103,38 @@ int parseq_forward_host(parseq_engine* e, const parseq_forward_args* args, const
 /* "Next" rows of the path (SURVEY.md section 8f).
  * Raw-crop input: images uint8 [N, H, W, 3] (HWC, as PIL / numpy hold them, already resized to img_size); the reference's
  * T.ToTensor() + T.Normalize(0.5, 0.5) (strhub/data/module.py:68-82) is folded into the patch gather.  Device / host
- * variants mirror parseq_forward / parseq_forward_host. */
+ * variants mirror parseq_forward / parseq_forward_host.  Crops of any size go through parseq_forward_crops below. */
 int parseq_forward_u8(parseq_engine* e, const parseq_forward_args* args, const uint8_t* images_hwc,
                       float* logits, int32_t* ids, int32_t* steps, parseq_stream_t stream);
 int parseq_forward_host_u8(parseq_engine* e, const parseq_forward_args* args, const uint8_t* images_hwc_host,
                            float* logits_host, int32_t* ids_host, int32_t* steps_host, parseq_stream_t stream);
+
+/* Variable-size RGB uint8 crops: the reference's whole input transform (strhub/data/module.py:69-82, read.py)
+ *   [img.rotate(rotation, expand=True)] -> T.Resize(img_size, BICUBIC) -> T.ToTensor() -> T.Normalize(0.5, 0.5)
+ * on the GPU.  The resize is bit-exact with PIL's bicubic resampler (what torchvision's Resize runs on PIL images), so
+ * the result is bit-identical to parseq_forward_u8 on the PIL-resized stack, for any batch.
+ * A crop is `height` rows of 3 * `width` bytes (R, G, B per pixel), row i starting at byte offset + i * row_stride of
+ * `pixels`; row_stride >= 3 * width, so a crop can be a view into a larger frame.  Each side is 1..4096 pixels; every
+ * crop must lie inside [0, pixels_bytes).  Anything else returns PARSEQ_ERR_INVALID_ARG before any work is enqueued. */
+typedef struct parseq_crop {
+  int64_t offset;
+  int32_t height, width, row_stride;
+  int32_t reserved;                      /* 0 */
+} parseq_crop;
+typedef struct parseq_crops {
+  int32_t count;                         /* == args->batch */
+  const parseq_crop* desc;               /* HOST array [count]; may be reused as soon as the call returns */
+  const uint8_t* pixels;                 /* packed RGB bytes: DEVICE for parseq_forward_crops, HOST for the _host variant */
+  int64_t pixels_bytes;                  /* the host variant uploads all of [0, pixels_bytes) */
+  int32_t rotation;                      /* 0, 90, 180, 270: counter-clockwise, expand=True (read.py / test.py --rotation) */
+} parseq_crops;
+int parseq_forward_crops(parseq_engine* e, const parseq_forward_args* args, const parseq_crops* crops, float* logits,
+                         int32_t* ids, int32_t* steps, parseq_stream_t stream);
+int parseq_forward_host_crops(parseq_engine* e, const parseq_forward_args* args, const parseq_crops* crops,
+                              float* logits_host, int32_t* ids_host, int32_t* steps_host, parseq_stream_t stream);
+/* The resize alone: out_hwc DEVICE uint8 [count, img_h, img_w, 3] (the input of parseq_forward_u8); crops->pixels is
+ * DEVICE.  Needs no weights. */
+int parseq_resize_crops(parseq_engine* e, const parseq_crops* crops, uint8_t* out_hwc, parseq_stream_t stream);
 /* Fused post-processing of BaseSystem._eval_step (strhub/models/base.py:132-142) + Tokenizer._filter
  * (strhub/data/utils.py:120-129): DEVICE logits [N, num_steps, num_classes] -> ids [N, num_steps] (greedy), lengths [N]
  * (index of the first EOS, num_steps if none) and confidence [N] (product of the max softmax probabilities up to and

@@ -10,7 +10,7 @@ CSRC = os.path.join(PKG, "csrc")
 LIB_DIR = os.path.join(PKG, "lib")
 LIB_PATH = os.path.join(LIB_DIR, "libparseq_b200.so")
 SOURCES = ["engine.cu"]
-HEADERS = ["ptx.cuh", "gemm.cuh", "kernels.cuh", "dec_ar.cuh", "dec_ar2.cuh", "attn_tc.cuh", "gemm_ln.cuh", "gemm_ln2.cuh", "mlp_ln.cuh", os.path.join("..", "..", "include", "parseq_b200.h")]
+HEADERS = ["ptx.cuh", "gemm.cuh", "kernels.cuh", "dec_ar.cuh", "dec_ar2.cuh", "attn_tc.cuh", "gemm_ln.cuh", "gemm_ln2.cuh", "mlp_ln.cuh", "resize.cuh", os.path.join("..", "..", "include", "parseq_b200.h")]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",

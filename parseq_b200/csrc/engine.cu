@@ -22,6 +22,7 @@
 #include "gemm_ln.cuh"
 #include "gemm_ln2.cuh"
 #include "mlp_ln.cuh"
+#include "resize.cuh"
 
 namespace {
 
@@ -613,6 +614,16 @@ struct parseq_engine {
   bool use_graph = true;
   struct GraphEntry { cudaGraphExec_t exec; long long kernels; };
   std::map<std::vector<int>, GraphEntry> graphs;
+  // crop entry points (resize.cuh): the plan of the current call, built on the host and uploaded to engine-owned
+  // buffers that grow on demand, plus the device staging copy of host pixels
+  std::vector<pq::RzCrop> rz_hcrops;
+  std::vector<pq::RzTask> rz_htasks;
+  std::vector<long long> rz_first;  // [count + 1] index of the first task of each crop
+  int rz_smem = 0;                  // dynamic shared memory of the plan's largest task
+  int rz_rot = 0;                   // rotation of the plan
+  pq::RzCrop* rz_crops = nullptr; long long rz_crops_cap = 0;
+  pq::RzTask* rz_tasks = nullptr; long long rz_tasks_cap = 0;
+  uint8_t* rz_stage = nullptr; long long rz_stage_cap = 0;
 
   void* w(const std::string& k) const { return slots[index.at(k)].dev; }
   const float* wf(const std::string& k) const { return reinterpret_cast<const float*>(w(k)); }
@@ -1330,9 +1341,162 @@ int run_graph(parseq_engine* e, const parseq_forward_args* a, int Bc, int L, boo
   return PARSEQ_OK;
 }
 
+// ---------------------------------------------------------------- variable-size crops (resize.cuh)
+constexpr int RZ_MAX_SIDE = 4096;
+constexpr int RZ_BAND = 8;                      // output rows per task at most
+constexpr int RZ_SMEM_BUDGET = 48 * 1024;       // per-task shared memory the planner aims for (several CTAs per SM)
+
+// shared memory of a task (the layout of resize_bicubic_u8_kernel)
+long long rz_task_bytes(int ny, int nx, int nr, int wcols, int kh, int kv) {
+  return 4ll * (2 * ny + 2 * nx + 1ll * ny * kv + 1ll * nx * kh) + 3ll * nr * wcols;
+}
+
+// Host copy of the kernel's first-tap / tap-count arithmetic (precompute_coeffs), used to size the row windows.
+void rz_bounds(int in_size, int out_size, std::vector<int>& xmin, std::vector<int>& cnt) {
+  xmin.resize(static_cast<size_t>(out_size));
+  cnt.resize(static_cast<size_t>(out_size));
+  if (in_size == out_size) {
+    for (int i = 0; i < out_size; ++i) { xmin[i] = i; cnt[i] = 1; }
+    return;
+  }
+  const double scale = static_cast<double>(in_size) / out_size;
+  const double support = 2.0 * (scale < 1.0 ? 1.0 : scale);
+  for (int xx = 0; xx < out_size; ++xx) {
+    const double center = (xx + 0.5) * scale;
+    int lo = static_cast<int>(center - support + 0.5);
+    if (lo < 0) lo = 0;
+    int hi = static_cast<int>(center + support + 0.5);
+    if (hi > in_size) hi = in_size;
+    xmin[xx] = lo;
+    cnt[xx] = hi - lo;
+  }
+}
+
+// Validates every crop, then splits each into tasks: (band of <= RZ_BAND output rows) x (tile of output columns) whose
+// shared memory fits RZ_SMEM_BUDGET where possible and the device limit always.  Changes nothing on failure.
+int rz_plan(parseq_engine* e, const parseq_crops* cr) {
+  if (cr == nullptr) return fail(PARSEQ_ERR_INVALID_ARG, "null crops");
+  if (cr->count < 0) return fail(PARSEQ_ERR_INVALID_ARG, "negative crop count");
+  if (cr->count > 0 && (cr->desc == nullptr || cr->pixels == nullptr))
+    return fail(PARSEQ_ERR_INVALID_ARG, "crops: null desc / pixels");
+  if (cr->rotation != 0 && cr->rotation != 90 && cr->rotation != 180 && cr->rotation != 270)
+    return fail(PARSEQ_ERR_INVALID_ARG, "crops: rotation must be 0, 90, 180 or 270, got " + std::to_string(cr->rotation));
+  if (cr->pixels_bytes < 0) return fail(PARSEQ_ERR_INVALID_ARG, "crops: negative pixels_bytes");
+  for (int i = 0; i < cr->count; ++i) {
+    const parseq_crop& d = cr->desc[i];
+    const std::string at = "crop " + std::to_string(i) + ": ";
+    if (d.height < 1 || d.width < 1 || d.height > RZ_MAX_SIDE || d.width > RZ_MAX_SIDE)
+      return fail(PARSEQ_ERR_INVALID_ARG, at + "size " + std::to_string(d.height) + "x" + std::to_string(d.width) +
+                                              " outside 1..4096");
+    if (d.row_stride < 3 * d.width) return fail(PARSEQ_ERR_INVALID_ARG, at + "row_stride < 3 * width");
+    if (d.offset < 0 || d.offset + 1ll * (d.height - 1) * d.row_stride + 3ll * d.width > cr->pixels_bytes)
+      return fail(PARSEQ_ERR_INVALID_ARG, at + "extends outside [0, pixels_bytes)");
+  }
+  int optin = 0, dev = 0;
+  PQ_CUDA(cudaGetDevice(&dev));
+  PQ_CUDA(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
+  const int H = e->cfg.img_h, W = e->cfg.img_w;
+  std::vector<pq::RzCrop> crops;
+  std::vector<pq::RzTask> tasks;
+  std::vector<long long> first;
+  crops.reserve(static_cast<size_t>(cr->count));
+  first.reserve(static_cast<size_t>(cr->count) + 1);
+  long long smem = 0;
+  std::vector<int> vmin, vcnt;
+  for (int i = 0; i < cr->count; ++i) {
+    const parseq_crop& d = cr->desc[i];
+    const bool turn = cr->rotation == 90 || cr->rotation == 270;
+    pq::RzCrop c{d.offset, d.height, d.width, d.row_stride, turn ? d.width : d.height, turn ? d.height : d.width, 0};
+    c.vfirst = (c.hr > 100 * c.wr && H < c.hr) ? 1 : 0;    // PIL Image.resize: very tall images shrink height first
+    const int kh = c.wr != W ? pq::rz_ksize(c.wr, W) : 0, kv = c.hr != H ? pq::rz_ksize(c.hr, H) : 0;
+    rz_bounds(c.hr, H, vmin, vcnt);
+    // window rows of output rows [y0, y1) and their width in pixels for a tile of nx columns
+    auto rows = [&](int y0, int y1) { return c.vfirst ? (y1 - y0) : (vmin[y1 - 1] + vcnt[y1 - 1] - vmin[y0]); };
+    auto bytes = [&](int y0, int y1, int nx) {
+      return rz_task_bytes(y1 - y0, nx, rows(y0, y1), c.vfirst ? c.wr : nx, kh, kv);
+    };
+    int max_rows = 0;
+    for (int y = 0; y < H; ++y) max_rows = std::max(max_rows, rows(y, y + 1));
+    auto one_row = [&](int nx) {
+      return rz_task_bytes(1, nx, c.vfirst ? 1 : max_rows, c.vfirst ? c.wr : nx, kh, kv);
+    };
+    const long long budget = std::max<long long>(RZ_SMEM_BUDGET, one_row(1));
+    if (budget > optin) return fail(PARSEQ_ERR_UNSUPPORTED, "crop " + std::to_string(i) + ": resize does not fit shared memory");
+    int tiles = 1;
+    while (one_row((W + tiles - 1) / tiles) > budget) ++tiles;
+    const int nx = (W + tiles - 1) / tiles;
+    first.push_back(static_cast<long long>(tasks.size()));
+    for (int y0 = 0; y0 < H;) {
+      int y1 = y0 + 1;
+      while (y1 < H && y1 - y0 < RZ_BAND && bytes(y0, y1 + 1, nx) <= budget) ++y1;
+      for (int x0 = 0; x0 < W; x0 += nx) {
+        const int n = std::min(nx, W - x0);
+        tasks.push_back(pq::RzTask{i, y0, y1 - y0, x0, n, c.vfirst ? 0 : vmin[y0], rows(y0, y1)});
+        smem = std::max(smem, bytes(y0, y1, n));
+      }
+      y0 = y1;
+    }
+    crops.push_back(c);
+  }
+  first.push_back(static_cast<long long>(tasks.size()));
+  e->rz_hcrops.swap(crops);
+  e->rz_htasks.swap(tasks);
+  e->rz_first.swap(first);
+  e->rz_smem = static_cast<int>((smem + 15) & ~15ll);
+  e->rz_rot = cr->rotation;
+  return PARSEQ_OK;
+}
+
+// Grows an engine-owned device buffer to hold n elements; on failure the old buffer is kept.
+template <typename Tp>
+int rz_reserve(parseq_engine* e, Tp** buf, long long* cap, long long n) {
+  if (n <= *cap) return PARSEQ_OK;
+  Tp* p = nullptr;
+  PQ_TRY(dev_alloc(&p, n));
+  PQ_CUDA(cudaStreamSynchronize(e->main));       // the old buffer may still be read by enqueued work
+  if (*buf) cudaFree(*buf);
+  *buf = p;
+  *cap = n;
+  return PARSEQ_OK;
+}
+
+// Validates and plans the crops, then uploads the plan (and, for host pixels, the pixels) on `main`.
+// Returns the device address of the pixels through *pixels_dev.
+int rz_prepare(parseq_engine* e, const parseq_crops* cr, bool host, const uint8_t** pixels_dev) {
+  PQ_TRY(rz_plan(e, cr));
+  PQ_TRY(rz_reserve(e, &e->rz_crops, &e->rz_crops_cap, std::max<long long>(1, cr->count)));
+  PQ_TRY(rz_reserve(e, &e->rz_tasks, &e->rz_tasks_cap, std::max<long long>(1, static_cast<long long>(e->rz_htasks.size()))));
+  if (host) PQ_TRY(rz_reserve(e, &e->rz_stage, &e->rz_stage_cap, std::max<long long>(16, cr->pixels_bytes)));
+  PQ_CUDA(cudaMemcpyAsync(e->rz_crops, e->rz_hcrops.data(), e->rz_hcrops.size() * sizeof(pq::RzCrop), cudaMemcpyHostToDevice,
+                          e->main));
+  PQ_CUDA(cudaMemcpyAsync(e->rz_tasks, e->rz_htasks.data(), e->rz_htasks.size() * sizeof(pq::RzTask), cudaMemcpyHostToDevice,
+                          e->main));
+  if (host && cr->pixels_bytes > 0)
+    PQ_CUDA(cudaMemcpyAsync(e->rz_stage, cr->pixels, static_cast<size_t>(cr->pixels_bytes), cudaMemcpyHostToDevice, e->main));
+  *pixels_dev = host ? e->rz_stage : cr->pixels;
+  return PARSEQ_OK;
+}
+
+// Resizes planned crops [b0, b0 + B) into out [B, img_h, img_w, 3].
+int rz_launch(parseq_engine* e, const uint8_t* pixels, int b0, int B, uint8_t* out, cudaStream_t st) {
+  static int smem_attr = 0;
+  if (e->rz_smem > smem_attr) {
+    PQ_CUDA(cudaFuncSetAttribute(pq::resize_bicubic_u8_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, e->rz_smem));
+    smem_attr = e->rz_smem;
+  }
+  const long long t0 = e->rz_first[static_cast<size_t>(b0)], t1 = e->rz_first[static_cast<size_t>(b0 + B)];
+  if (t1 == t0) return PARSEQ_OK;
+  TimedScope ts(e, st, CAT_MISC, 0.0);
+  return launch_k(e->lo, pq::resize_bicubic_u8_kernel, dim3(static_cast<unsigned>(t1 - t0)), dim3(pq::RZ_THREADS),
+                  static_cast<size_t>(e->rz_smem), st, pixels, static_cast<const pq::RzCrop*>(e->rz_crops),
+                  static_cast<const pq::RzTask*>(e->rz_tasks + t0), b0, out, e->cfg.img_h, e->cfg.img_w, e->rz_rot);
+}
+
 // Common driver of parseq_forward / parseq_forward_host. `host` selects H2D/D2H vs D2D staging copies.
+// crop_pixels != NULL (crop entry points, plan uploaded by rz_prepare): each super-chunk is resized into the uint8 input
+// buffer instead of copied there, then runs exactly as parseq_forward_u8 would.
 int forward_impl(parseq_engine* e, const parseq_forward_args* a, const void* images_any, float* logits, int32_t* ids,
-                 int32_t* steps, cudaStream_t user, bool host, bool u8 = false) {
+                 int32_t* steps, cudaStream_t user, bool host, bool u8 = false, const uint8_t* crop_pixels = nullptr) {
   const int L = num_steps_of(e, a->max_length);
   const bool testing = a->max_length < 0;
   const long long img_sz = 3ll * e->cfg.img_h * e->cfg.img_w * (u8 ? 1 : 4);   // bytes per image
@@ -1349,12 +1513,12 @@ int forward_impl(parseq_engine* e, const parseq_forward_args* a, const void* ima
   e->launches++;
   for (int b0 = 0; b0 < a->batch; b0 += e->max_batch) {
     const int Bc = (a->batch - b0 < e->max_batch) ? (a->batch - b0) : e->max_batch;
-    if (eager && !host) {
+    if (eager && !host && crop_pixels == nullptr) {
       PQ_TRY(forward_super(e, a, b0, Bc, L, images + b0 * img_sz, u8, logits + 1ll * b0 * L * e->C,
                            ids ? ids + 1ll * b0 * L : nullptr, e->out_steps));
       continue;
     }
-    if (host && !eager && e->arch == 0 && Bc >= 256 && e->chunk >= Bc) {
+    if (host && !eager && e->arch == 0 && Bc >= 256 && e->chunk >= Bc && crop_pixels == nullptr) {
       // upload in two halves on the copy stream; the encoder of the first half (its own graph) runs under the second upload
       const int split = ((Bc / 2 + 7) / 8) * 8;
       PQ_CUDA(cudaEventRecord(e->ev_c[2], e->main));                       // previous work on `main` (and the caller's stream)
@@ -1373,7 +1537,10 @@ int forward_impl(parseq_engine* e, const parseq_forward_args* a, const void* ima
       if (ids) PQ_CUDA(cudaMemcpyAsync(ids + 1ll * b0 * L, e->out_ids, static_cast<size_t>(1ll * Bc * L) * 4, kout, e->main));
       continue;
     }
-    PQ_CUDA(cudaMemcpyAsync(in_static, images + b0 * img_sz, static_cast<size_t>(Bc * img_sz), kin, e->main));
+    if (crop_pixels != nullptr)
+      PQ_TRY(rz_launch(e, crop_pixels, b0, Bc, e->in_images_u8, e->main));
+    else
+      PQ_CUDA(cudaMemcpyAsync(in_static, images + b0 * img_sz, static_cast<size_t>(Bc * img_sz), kin, e->main));
     if (eager) {
       PQ_TRY(forward_super(e, a, b0, Bc, L, in_static, u8, e->out_logits, e->out_ids, e->out_steps));
     } else {
@@ -1548,6 +1715,8 @@ void parseq_destroy(parseq_engine* e) {
   if (e->kvtab) cudaFree(e->kvtab);
   if (e->qs) cudaFree(e->qs);
   free_workspace(e);
+  for (void* p : {static_cast<void*>(e->rz_crops), static_cast<void*>(e->rz_tasks), static_cast<void*>(e->rz_stage)})
+    if (p) cudaFree(p);
   if (e->main) cudaStreamDestroy(e->main);
   if (e->copy) cudaStreamDestroy(e->copy);
   for (auto ev : e->ev_c) if (ev) cudaEventDestroy(ev);
@@ -1689,6 +1858,55 @@ int parseq_forward_host_u8(parseq_engine* e, const parseq_forward_args* a, const
   PQ_CUDA(cudaSetDevice(e->cfg.device));
   PQ_TRY(forward_impl(e, a, images_hwc_host, logits_host, ids_host, steps_host, reinterpret_cast<cudaStream_t>(stream), true, true));
   PQ_CUDA(cudaStreamSynchronize(e->main));
+  return PARSEQ_OK;
+}
+
+int parseq_forward_crops(parseq_engine* e, const parseq_forward_args* a, const parseq_crops* crops, float* logits, int32_t* ids,
+                         int32_t* steps, parseq_stream_t stream) {
+  if (e == nullptr || a == nullptr || crops == nullptr || logits == nullptr)
+    return fail(PARSEQ_ERR_INVALID_ARG, "null argument");
+  if (e->broken) return fail(PARSEQ_ERR_STATE, "engine workspace is gone (a failed resize): destroy the handle");
+  if (!e->finalized) return fail(PARSEQ_ERR_STATE, "parseq_finalize has not been called after the last weight update");
+  if (a->batch < 0 || a->refine_iters < 0) return fail(PARSEQ_ERR_INVALID_ARG, "negative batch / refine_iters");
+  if (crops->count != a->batch) return fail(PARSEQ_ERR_INVALID_ARG, "crops->count != args->batch");
+  PQ_CUDA(cudaSetDevice(e->cfg.device));
+  const uint8_t* px = nullptr;
+  PQ_TRY(rz_prepare(e, crops, false, &px));
+  if (a->batch == 0) return PARSEQ_OK;
+  return forward_impl(e, a, nullptr, logits, ids, steps, reinterpret_cast<cudaStream_t>(stream), false, true, px);
+}
+
+int parseq_forward_host_crops(parseq_engine* e, const parseq_forward_args* a, const parseq_crops* crops, float* logits_host,
+                              int32_t* ids_host, int32_t* steps_host, parseq_stream_t stream) {
+  if (e == nullptr || a == nullptr || crops == nullptr || logits_host == nullptr)
+    return fail(PARSEQ_ERR_INVALID_ARG, "null argument");
+  if (e->broken) return fail(PARSEQ_ERR_STATE, "engine workspace is gone (a failed resize): destroy the handle");
+  if (!e->finalized) return fail(PARSEQ_ERR_STATE, "parseq_finalize has not been called after the last weight update");
+  if (a->batch < 0 || a->refine_iters < 0) return fail(PARSEQ_ERR_INVALID_ARG, "negative batch / refine_iters");
+  if (crops->count != a->batch) return fail(PARSEQ_ERR_INVALID_ARG, "crops->count != args->batch");
+  if (a->forced_ids != nullptr || a->forced_refine != nullptr)
+    return fail(PARSEQ_ERR_INVALID_ARG, "teacher forcing is a device-pointer API (parseq_forward)");
+  PQ_CUDA(cudaSetDevice(e->cfg.device));
+  const uint8_t* px = nullptr;
+  PQ_TRY(rz_prepare(e, crops, true, &px));
+  if (a->batch == 0) return PARSEQ_OK;
+  PQ_TRY(forward_impl(e, a, nullptr, logits_host, ids_host, steps_host, reinterpret_cast<cudaStream_t>(stream), true, true, px));
+  PQ_CUDA(cudaStreamSynchronize(e->main));
+  return PARSEQ_OK;
+}
+
+int parseq_resize_crops(parseq_engine* e, const parseq_crops* crops, uint8_t* out_hwc, parseq_stream_t stream) {
+  if (e == nullptr || crops == nullptr || out_hwc == nullptr) return fail(PARSEQ_ERR_INVALID_ARG, "null argument");
+  PQ_CUDA(cudaSetDevice(e->cfg.device));
+  const uint8_t* px = nullptr;
+  PQ_TRY(rz_prepare(e, crops, false, &px));
+  if (crops->count == 0) return PARSEQ_OK;
+  cudaStream_t user = reinterpret_cast<cudaStream_t>(stream);
+  PQ_CUDA(cudaEventRecord(e->ev_in, user));
+  PQ_CUDA(cudaStreamWaitEvent(e->main, e->ev_in, 0));
+  PQ_TRY(rz_launch(e, px, 0, crops->count, out_hwc, e->main));
+  PQ_CUDA(cudaEventRecord(e->ev_out, e->main));
+  PQ_CUDA(cudaStreamWaitEvent(user, e->ev_out, 0));
   return PARSEQ_OK;
 }
 

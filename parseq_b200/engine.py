@@ -23,12 +23,22 @@ class ForwardArgsC(C.Structure):
                 ("refine_iters", C.c_int32), ("forced_ids", C.c_void_p), ("forced_refine", C.c_void_p)]
 
 
+class CropC(C.Structure):
+    _fields_ = [("offset", C.c_int64), ("height", C.c_int32), ("width", C.c_int32), ("row_stride", C.c_int32),
+                ("reserved", C.c_int32)]
+
+
+class CropsC(C.Structure):
+    _fields_ = [("count", C.c_int32), ("desc", C.POINTER(CropC)), ("pixels", C.c_void_p), ("pixels_bytes", C.c_int64),
+                ("rotation", C.c_int32)]
+
+
 EXPORTS = [
     "parseq_create", "parseq_destroy", "parseq_set_weight", "parseq_num_weights", "parseq_weight_key",
     "parseq_finalize", "parseq_forward", "parseq_forward_host", "parseq_forward_u8", "parseq_forward_host_u8",
     "parseq_postprocess", "parseq_encode", "parseq_decode", "parseq_head", "parseq_text_embed", "parseq_kernel_launches", "parseq_debug_int", "parseq_bench_tma_stream",
     "parseq_set_option", "parseq_get_timing", "parseq_get_ar_profile", "parseq_last_error", "parseq_version", "parseq_gemm_bf16", "parseq_gemm_ln_bf16", "parseq_mlp_ln_bf16", "parseq_mlp_ln_bf16_prof", "parseq_layernorm_bf16",
-    "parseq_enc_attention",
+    "parseq_enc_attention", "parseq_forward_crops", "parseq_forward_host_crops", "parseq_resize_crops",
 ]
 
 
@@ -61,6 +71,10 @@ def load_library(path: Optional[str] = None):
     lib.parseq_forward_host.argtypes = lib.parseq_forward.argtypes
     lib.parseq_forward_u8.argtypes = lib.parseq_forward.argtypes
     lib.parseq_forward_host_u8.argtypes = lib.parseq_forward.argtypes
+    lib.parseq_forward_crops.argtypes = [C.c_void_p, C.POINTER(ForwardArgsC), C.POINTER(CropsC), C.c_void_p, C.c_void_p,
+                                         C.c_void_p, C.c_void_p]
+    lib.parseq_forward_host_crops.argtypes = lib.parseq_forward_crops.argtypes
+    lib.parseq_resize_crops.argtypes = [C.c_void_p, C.POINTER(CropsC), C.c_void_p, C.c_void_p]
     lib.parseq_postprocess.argtypes = [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p,
                                        C.c_void_p, C.c_void_p]
     lib.parseq_encode.argtypes = [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]
@@ -197,6 +211,18 @@ class Engine:
         a = self._args(batch, max_length, decode_ar, refine_iters)
         fn = self.lib.parseq_forward_host_u8 if host else self.lib.parseq_forward_u8
         check(self.lib, fn(self.handle, C.byref(a), images_ptr, logits_ptr, ids_ptr, steps_ptr, stream))
+
+    def forward_crops(self, crops, logits_ptr, ids_ptr, steps_ptr, stream, max_length=None, decode_ar=True,
+                      refine_iters=1):
+        """`crops`: a `parseq_b200.crops.PackedCrops`; host pixels run parseq_forward_host_crops (host outputs,
+        synchronised on return), device pixels parseq_forward_crops (device outputs, enqueued on `stream`)."""
+        a = self._args(crops.count, max_length, decode_ar, refine_iters)
+        fn = self.lib.parseq_forward_host_crops if crops.host else self.lib.parseq_forward_crops
+        check(self.lib, fn(self.handle, C.byref(a), C.byref(crops.c_struct()), logits_ptr, ids_ptr, steps_ptr, stream))
+
+    def resize_crops(self, crops, out_ptr, stream):
+        """Device crops -> uint8 [count, img_h, img_w, 3] at `out_ptr` (device)."""
+        check(self.lib, self.lib.parseq_resize_crops(self.handle, C.byref(crops.c_struct()), out_ptr, stream))
 
     def postprocess(self, logits_ptr, batch, num_steps, ids_ptr, lengths_ptr, conf_ptr, stream, eos_id=0):
         check(self.lib, self.lib.parseq_postprocess(logits_ptr, batch, num_steps, self.cfg.num_classes, eos_id, ids_ptr,

@@ -211,6 +211,30 @@ class _EngineModule(nn.Module):
                         fr.data_ptr() if fr is not None else None)
         return logits, ids, steps
 
+    def _run_crops(self, crops, max_length, decode_ar, refine_iters, rotation):
+        """Variable-size RGB crops (see parseq_b200.crops): rotate + bicubic resize + normalise on the GPU, then the
+        uint8 path.  Outputs are on the model's device whatever the crops' location."""
+        from .crops import PackedCrops, pack_crops
+        eng = self.engine()
+        packed = crops if isinstance(crops, PackedCrops) else pack_crops(crops, rotation)
+        dev = self._device
+        N, L = packed.count, eng.num_steps(max_length)
+        shapes = ((N, L, self.cfg.num_classes), (N, L), (1,))
+        if not packed.host and packed.device != dev:
+            raise RuntimeError(f"crops are on {packed.device}, the model on {dev}")
+        pin = packed.host
+        where = dict(pin_memory=True) if pin else dict(device=dev)
+        logits, ids, steps = (torch.empty(shp, dtype=dt, **where)
+                              for shp, dt in zip(shapes, (torch.float32, torch.int32, torch.int32)))
+        if N == 0:
+            steps.fill_(L)
+        else:
+            eng.forward_crops(packed, logits.data_ptr(), ids.data_ptr(), steps.data_ptr(),
+                              torch.cuda.current_stream(dev).cuda_stream, max_length, decode_ar, refine_iters)
+        if pin:             # the host entry point returns synchronised host results
+            logits, ids, steps = (t.to(dev, non_blocking=True) for t in (logits, ids, steps))
+        return logits, ids, steps
+
 
 class ParseqModel(_EngineModule):
     def __init__(self, cfg: ParseqConfig):
@@ -272,6 +296,17 @@ class ParseqModel(_EngineModule):
                 return_ids: bool = False, forced_ids: Optional[Tensor] = None,
                 forced_refine: Optional[Tensor] = None):
         logits, ids, steps = self._run(images, max_length, self.decode_ar, self.refine_iters, forced_ids, forced_refine)
+        return self._finish(logits, ids, steps, max_length, return_ids)
+
+    def forward_crops(self, tokenizer: Tokenizer, crops, max_length: Optional[int] = None, rotation: int = 0,
+                      return_ids: bool = False):
+        """`forward` on variable-size RGB crops (PIL images, uint8 numpy / torch [h, w, 3], or a PackedCrops) with the
+        reference's input transform - rotate(rotation, expand=True), Resize(img_size, BICUBIC), ToTensor, Normalize -
+        run on the GPU; bit-identical to `forward` on the uint8 stack PIL's resize produces."""
+        logits, ids, steps = self._run_crops(crops, max_length, self.decode_ar, self.refine_iters, rotation)
+        return self._finish(logits, ids, steps, max_length, return_ids)
+
+    def _finish(self, logits, ids, steps, max_length, return_ids):
         if max_length is None and self.decode_ar and not self.refine_iters:
             # model.py:144-147: with no refinement the reference returns only the S steps it ran
             S = int(steps.item())
@@ -291,6 +326,11 @@ class VitstrModel(_EngineModule):
     def forward_tokens(self, images: Tensor, max_length: Optional[int] = None, return_ids: bool = False):
         """`self.forward(images, max_length + 2)[:, 1:]` (vitstr/system.py:65-71) in one engine call."""
         logits, ids, _ = self._run(images, max_length, False, 0)
+        return (logits, ids) if return_ids else logits
+
+    def forward_tokens_crops(self, crops, max_length: Optional[int] = None, rotation: int = 0, return_ids: bool = False):
+        """`forward_tokens` on variable-size RGB crops (see ParseqModel.forward_crops)."""
+        logits, ids, _ = self._run_crops(crops, max_length, False, 0, rotation)
         return (logits, ids) if return_ids else logits
 
     def forward(self, x: Tensor, seqlen: int = 25) -> Tensor:
@@ -338,6 +378,10 @@ class _System(nn.Module):
         ids_h, len_h, conf_h = ids.cpu().tolist(), lengths.cpu().tolist(), conf.cpu().tolist()
         labels = [self.tokenizer._ids2tok(row[:n], True) for row, n in zip(ids_h, len_h)]
         return labels, conf_h
+
+    def read(self, crops, rotation: int = 0):
+        """The reference's read.py in one call: variable-size RGB crops -> (labels, confidences)."""
+        return self.postprocess(self.forward_crops(crops, rotation=rotation))
 
     # base.py:112-143,179-180 (test path only; validation loss is a training concern)
     def _eval_step(self, batch, validation: bool = False):
@@ -403,6 +447,10 @@ class PARSeq(_System):
     def forward(self, images: Tensor, max_length: Optional[int] = None) -> Tensor:
         return self.model.forward(self.tokenizer, images, max_length)
 
+    def forward_crops(self, crops, max_length: Optional[int] = None, rotation: int = 0) -> Tensor:
+        """`forward` on variable-size RGB crops, resized on the GPU exactly as T.Resize(img_size, BICUBIC) does."""
+        return self.model.forward_crops(self.tokenizer, crops, max_length, rotation)
+
 
 class ViTSTR(_System):
     """Mirror of `strhub.models.vitstr.system.ViTSTR` (vitstr/system.py:29-71), inference side."""
@@ -431,6 +479,10 @@ class ViTSTR(_System):
 
     def forward(self, images: Tensor, max_length: Optional[int] = None) -> Tensor:
         return self.model.forward_tokens(images, max_length)
+
+    def forward_crops(self, crops, max_length: Optional[int] = None, rotation: int = 0) -> Tensor:
+        """`forward` on variable-size RGB crops, resized on the GPU exactly as T.Resize(img_size, BICUBIC) does."""
+        return self.model.forward_tokens_crops(crops, max_length, rotation)
 
     @classmethod
     def load_from_checkpoint(cls, checkpoint_path: str, map_location="cpu", **kwargs):
